@@ -370,6 +370,28 @@ def c3_probe_leg(pkg, torch, dev, local_rank, chains=262144, draws=10):
         return {"error": "%s: %s" % (type(e).__name__, str(e)[:300])}
 
 
+DUMP_BYTES = 60 << 20
+
+
+def dump_outputs(out_dir, draws, stats, logd, stats_dtype):
+    """What the last timed step handed its caller, as float64 .npy files: posterior_matrix [m, n, D], logdensities [m, n]
+    and one tree_statistics_<field> [m, n] per field, for m chains: all of them, or a fixed seeded sample when all would
+    exceed DUMP_BYTES; chains.npy holds their indices."""
+    import torch
+    K, n, D = draws.shape
+    m = min(K, max(1, DUMP_BYTES // (8 * (n * (D + 8) + 1))))
+    idx = np.arange(K) if m == K else np.sort(np.random.default_rng(0).choice(K, m, replace=False))
+    sel = torch.from_numpy(idx).to(draws.device)
+    st = stats.index_select(0, sel).cpu().numpy().view(stats_dtype)[..., 0]
+    arrays = {"chains": idx, "posterior_matrix": draws.index_select(0, sel).cpu().numpy(),
+              "logdensities": logd.index_select(0, sel).cpu().numpy()}
+    for f in ("pi", "depth", "left", "right", "acceptance_rate", "steps", "directions"):
+        arrays["tree_statistics_" + f] = st[f]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -388,6 +410,8 @@ def main():
     ap.add_argument("--ref-seconds", type=float, default=1.2)
     ap.add_argument("--cpu-baseline-seconds", type=float, default=4.0)
     ap.add_argument("--skip-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (rank 0's chains) to DIR/<name>.npy, at most 64 MB")
     args = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -459,6 +483,8 @@ def main():
     wall = time.perf_counter() - t0
     clocks = sampler.stop()
     launches = eng.kernel_launches() - launches0
+    if args.dump_outputs and rank == 0:      # before the legs below, which reuse these buffers
+        dump_outputs(args.dump_outputs, draws, stats, logd, pkg._lib.tree_stats_dtype)
     summary = eng.tree_summary_dev(stats.data_ptr(), n, ebfmi=False) if rank == 0 else None
     q_typical = None if args.skip_e2e else eng.get_state(("q",))["q"]   # posterior draws: the e2e steps start from them
 

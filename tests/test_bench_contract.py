@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -34,13 +36,16 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
-def test_b200_arm_orchestration_emits_one_contract_line_with_stub_engine():
+def test_b200_arm_orchestration_emits_one_contract_line_with_stub_engine(tmp_path):
     """The b200 arm cannot run without a GPU; its ORCHESTRATION can: tests/bench_stub_driver.py replaces torch's CUDA entry
     points and the engine by stand-ins and runs bench.main() with the default configuration.  Checked: exactly one JSON line on
-    stdout with every key of the contract, the roofline / cpu_baseline / e2e objects, and the three auxiliary legs
-    (user_model, c4_probe, c3_probe) present without an error.  (The numbers are the stand-in's and mean nothing.)"""
+    stdout with every key of the contract, the roofline / cpu_baseline / e2e objects, the three auxiliary legs
+    (user_model, c4_probe, c3_probe) present without an error, and the --dump-outputs files (names, shapes, dtype, size).
+    (The numbers are the stand-in's and mean nothing.)"""
+    dump = tmp_path / "dump"
     out = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "bench_stub_driver.py"), "--steps", "2", "--warmup", "3",
-                          "--cpu-baseline-seconds", "0.2"], capture_output=True, text=True, timeout=600, cwd=ROOT)
+                          "--cpu-baseline-seconds", "0.2", "--dump-outputs", str(dump)],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-3000:]
     lines = [l for l in out.stdout.splitlines() if l.strip()]
     assert len(lines) == 1
@@ -58,3 +63,12 @@ def test_b200_arm_orchestration_emits_one_contract_line_with_stub_engine():
     for leg in ("user_model", "c4_probe", "c3_probe"):
         assert leg in r and "error" not in r[leg] and r[leg]["value"] > 0 and r[leg]["unit"] == r["unit"], (leg, r.get(leg))
     assert r["user_model"]["model"] == "std_normal_user" and r["user_model"]["same_trees"] is True
+    fields = ("pi", "depth", "left", "right", "acceptance_rate", "steps", "directions")
+    names = {"chains", "posterior_matrix", "logdensities"} | {"tree_statistics_" + f for f in fields}
+    assert {p.name for p in dump.iterdir()} == {n + ".npy" for n in names}
+    a = {n: np.load(dump / (n + ".npy")) for n in names}
+    assert all(v.dtype == np.float64 for v in a.values())
+    assert sum(p.stat().st_size for p in dump.iterdir()) <= 64 << 20
+    m = a["chains"].size                                    # a seeded sample: 65 536 chains x 2 draws x 1000 dims is 1 GB
+    assert 1000 < m < 65536 and np.all(np.diff(a["chains"]) > 0) and a["chains"][-1] < 65536
+    assert a["posterior_matrix"].shape == (m, 2, 1000) and all(a[n].shape == (m, 2) for n in names - {"chains", "posterior_matrix"})
